@@ -1,6 +1,6 @@
 """bench.py - learner frames/sec of the B200-native IMPALA learner hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one full learn() step (AtariNet forward, fused V-trace + losses + their gradients,
@@ -17,6 +17,8 @@ Printed JSON (one line, rank 0):
   roofline / roofline_ops / vtrace / cpu_baseline / clocks / gpu_launches: see DESIGN.md section 5.
 `--impl reference` times the CPU restatement of the reference's learner step (oracle/, kind
 "port") on the host cores: the reference itself is PyTorch-on-CPU code that cannot travel to the box.
+`--dump-outputs DIR` saves what the last timed device-resident step returned, plus the updated parameters, as
+DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -58,7 +60,15 @@ def parse():
                     help="BASELINE configs[2]: N synthetic host actor threads -> pinned slots -> learner queue -> "
                          "polybeast_learner.learn on --learner_threads threads; prints the end-to-end SPS line")
     ap.add_argument("--learner_threads", type=int, default=2)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save what the last device-resident step computed as DIR/<name>.npy "
+                         "(float32, at most 64 MB in all); the inputs depend only on the arguments")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.actors > 0 or args.impl == "reference"):
+        ap.error("--dump-outputs saves the device-resident learn step; it does not apply to --actors or --impl reference")
+    return args
 
 
 # what the arithmetic is, per backend (the line's `dtype`)
@@ -268,6 +278,31 @@ def gemm_bytes_table(N, A, use_lstm, precision):
                   "lstm_wgrad": 4 * (N * 4 * H * e + N * H * e + 4 * H * H * 4),
                   "lstm_xproj_dgrad": 2 * (N * 4 * H * e + 4 * H * H * e + N * H * 4)})
     return t
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(out, model):
+    """Host copies of what one learn step hands its caller: the fused loss kernel's outputs (losses, V-trace targets,
+    policy-gradient advantages, log-rhos, action log-probs, loss gradients) and the updated flat parameters (the actor's
+    copy is identical)."""
+    arrays = dict(out["vtrace"]._asdict(), params=model.flat_params)
+    return {k: v.detach().cpu().numpy() for k, v in arrays.items() if v is not None}
+
+
+def write_outputs(arrays, out_dir, limit=DUMP_LIMIT_BYTES):
+    """Save each array as out_dir/<name>.npy in float32 (float64 stays float64).  When together they exceed `limit`
+    bytes, each array above an even share of it is stored as a sample of its flattened elements at sorted positions
+    drawn from RandomState(0): the same arguments give the same positions, so two builds can be compared."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32) for k, a in arrays.items()}
+    share = limit // max(len(arrays), 1) - 4096  # room for each file's .npy header
+    sample = sum(a.nbytes + 4096 for a in arrays.values()) > limit
+    for name, a in arrays.items():
+        if sample and a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, share // a.itemsize, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def resnet_flops_table(N, A):
@@ -632,6 +667,8 @@ def main():
     clocks = sampler.stop(t_region0, time.time()) if sampler else None
     final_loss = float(out["losses"][3])
     assert np.isfinite(final_loss), "non-finite loss"
+    if args.dump_outputs and rank == 0:  # before any further step overwrites the outputs or the parameters
+        write_outputs(step_outputs(out, model), args.dump_outputs)
     if graphed is not None:  # launches per step: count one eager step (a graph replay launches the same kernels)
         l0 = lib.tb_launch_count()
         learner.learn_step(flags, model, actor, devb[0], state, opt, None, stats_sync=False)

@@ -1,9 +1,12 @@
-"""Host-side pieces of bench.py that can be checked without a GPU: the clock sampler's parsing / time-window filter."""
+"""Host-side pieces of bench.py that can be checked without a GPU: the clock sampler's parsing / time-window filter and
+the --dump-outputs writer."""
 import datetime
 import importlib.util
 import os
 import sys
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -57,3 +60,31 @@ def test_clock_sampler_survives_garbage():
     s.rows = [["not a timestamp", "1950", "1965", "1", "Not Active", "Not Active", "Not Active", "Not Active"]]
     out = s.stop(now, now + 0.1)
     assert out["samples"] == 1 and out["in_timed_region"] is False
+
+
+def test_write_outputs_keeps_small_arrays_whole(tmp_path):
+    b = _bench()
+    arrays = dict(losses=np.arange(4, dtype=np.float32), vs=np.ones((3, 2), np.float64), act=np.arange(6).reshape(2, 3))
+    b.write_outputs(arrays, str(tmp_path / "out"))
+    got = {f[:-4]: np.load(str(tmp_path / "out" / f)) for f in os.listdir(str(tmp_path / "out"))}
+    assert sorted(got) == ["act", "losses", "vs"]
+    assert got["vs"].dtype == np.float64 and got["losses"].dtype == np.float32 and got["act"].dtype == np.float32
+    for k, a in arrays.items():
+        np.testing.assert_array_equal(got[k], a)
+
+
+def test_write_outputs_samples_to_the_limit_at_fixed_positions(tmp_path):
+    b = _bench()
+    rs = np.random.RandomState(1)
+    arrays = dict(params=rs.randn(300000).astype(np.float32), grads=rs.randn(50, 40, 30).astype(np.float32),
+                  losses=np.arange(4, dtype=np.float32))
+    limit = 3 * 4096 + 3 * 100000
+    for d in ("a", "b"):
+        b.write_outputs(arrays, str(tmp_path / d), limit=limit)
+    files = sorted(os.listdir(str(tmp_path / "a")))
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in files) <= limit
+    for f in files:
+        np.testing.assert_array_equal(np.load(str(tmp_path / "a" / f)), np.load(str(tmp_path / "b" / f)))
+    np.testing.assert_array_equal(np.load(str(tmp_path / "a" / "losses.npy")), arrays["losses"])
+    p = np.load(str(tmp_path / "a" / "params.npy"))
+    assert p.size == 100000 // 4 and np.isin(p, arrays["params"]).all()
